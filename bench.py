@@ -81,7 +81,12 @@ def parse():
     ap.add_argument("--cpu-frames", type=int, default=0, help="frame-steps per CPU sample (0 = sized from the time budget)")
     ap.add_argument("--no-extras", action="store_true", help="skip the side measurements (other batch sizes, 0.6B, encoders)")
     ap.add_argument("--no-parity-check", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy "
+                    "(waveforms and codes, float32), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def _pin(t):
@@ -413,6 +418,25 @@ def voice_clone_probe(eng, q, cfg, W, args, spk, B, N, dev):
             "h2d_bytes": int(wav_h.numel() * 4 + text_h.numel() * 2), "d2h_bytes": int(B * shape[-1] * 4)}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, wav, codes):
+    """The last timed step's waveforms (B, N*1920) and codes (B, N, 16) as float32 .npy files (7.7 MB + 64 KB at the
+    default shape).  Waveforms that would take the dump past DUMP_BYTES are cut to a fixed, seeded sample of time
+    positions, the same for every row, written beside them as wav_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    codes = codes.float().cpu().numpy()
+    wav = wav.float().reshape(wav.shape[0], -1).cpu().numpy()
+    keep = (DUMP_BYTES - codes.nbytes - 4096) // (4 * wav.shape[0] + 8)   # a float32 per row and a float64 index per position, .npy headers
+    if wav.shape[1] > keep:
+        idx = np.sort(np.random.default_rng(0).choice(wav.shape[1], keep, replace=False))
+        wav = wav[:, idx]
+        np.save(os.path.join(out_dir, "wav_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "wav.npy"), wav)
+    np.save(os.path.join(out_dir, "codes.npy"), codes)
+
+
 def hbm_peak():
     peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(peaks_path):
@@ -539,7 +563,7 @@ def main():
         if timed:
             torch.cuda.synchronize()
             t_pre += e0.elapsed_time(e1); t_dec += e1.elapsed_time(e2); t_cod += e2.elapsed_time(e3)
-        return wav
+        return wav, codes
 
     for _ in range(args.warmup):
         step_resident(False)
@@ -549,7 +573,7 @@ def main():
     s0, s1 = ev(), ev()
     s0.record(stream)
     for _ in range(args.steps):
-        wav = step_resident(True)
+        wav, codes = step_resident(True)
     s1.record(stream)
     barrier()
     ms_total = s0.elapsed_time(s1)
@@ -557,6 +581,8 @@ def main():
     fd, n_valid, _ = eng.ar.progress()
     assert fd == N and all(v == N for v in n_valid), (fd, n_valid)
     assert torch.isfinite(wav).all()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, wav, codes)
 
     # ---- end-to-end through the public calls: pinned host inputs, H2D + D2H inside the timed region.  The global
     # request list (B per GPU) goes through parallel.run_data_parallel: shard -> synthesize -> gather of waveforms

@@ -2,6 +2,9 @@
 (config.json + [sharded] safetensors + speech_tokenizer/ + generation_config.json) must load into exactly the config
 records and state_dict the engines are built from.  CPU only (no engine is constructed here)."""
 import dataclasses
+import json
+import os
+import types
 
 import pytest
 import torch
@@ -51,31 +54,34 @@ def test_config_defaults_and_errors(tmp_path):
         checkpoint.read_state_dict(str(tmp_path))
 
 
-@pytest.mark.reference
+def _reference_configs():
+    """The reference's config classes as oracle/make_golden.py recorded them: to_dict() of the tiny checkpoint's
+    configs, and the attributes of those objects and of default-constructed ones."""
+    from oracle.make_golden import from_json
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_configs.json")) as f:
+        return json.load(f, object_hook=from_json)
+
+
 def test_config_dict_matches_reference_config_classes():
     """The reference's own config classes, serialised with to_dict(), must map to the same records as from_hf()."""
-    from oracle import ref_shims
-    ref_shims.install()
-    from qwen_tts.core.models.configuration_qwen3_tts import Qwen3TTSConfig
     from qwen3_tts_b200 import checkpoint
     from qwen3_tts_b200.config import TTSConfig
-    top, _, _ = tiny_checkpoint_configs()
-    kw = {k: v for k, v in top.items() if k != "model_type"}
-    kw["talker_config"] = dict(kw["talker_config"], pad_token_id=None)
-    kw["talker_config"]["code_predictor_config"] = dict(kw["talker_config"]["code_predictor_config"], pad_token_id=None)
-    ref = Qwen3TTSConfig(**kw)
-    via_dict, meta = checkpoint.tts_config_from_dict(ref.to_dict())
+    R = _reference_configs()
+    ref = types.SimpleNamespace(**R["tts"]["top"])
+    ref.talker_config = types.SimpleNamespace(**R["tts"]["talker"])
+    ref.talker_config.code_predictor_config = types.SimpleNamespace(**R["tts"]["cp"])
+    via_dict, meta = checkpoint.tts_config_from_dict(R["tts_to_dict"])
     assert dataclasses.asdict(via_dict) == dataclasses.asdict(TTSConfig.from_hf(ref))
     assert meta["spk_id"] == ref.talker_config.spk_id
     # defaults table == the reference's constructor defaults
-    d = Qwen3TTSConfig(talker_config=dict(pad_token_id=None, code_predictor_config=dict(pad_token_id=None)))
+    d = R["tts_defaults"]
     # (rope_scaling is skipped: transformers 5.x rewrites None into {"rope_type": "default", ...} on construction)
     for k, v in checkpoint.TALKER_DEFAULTS.items():
-        assert k == "rope_scaling" or getattr(d.talker_config, k) == v, k
+        assert k == "rope_scaling" or d["talker"][k] == v, k
     for k, v in checkpoint.CODE_PREDICTOR_DEFAULTS.items():
-        assert k == "rope_scaling" or getattr(d.talker_config.code_predictor_config, k) == v, k
+        assert k == "rope_scaling" or d["cp"][k] == v, k
     for k, v in checkpoint.TOP_DEFAULTS.items():
-        assert getattr(d, k) == v, k
+        assert d["top"][k] == v, k
 
 
 def test_from_pretrained_plumbing_with_stub_engines(tmp_path, monkeypatch):
@@ -133,22 +139,15 @@ def test_from_pretrained_plumbing_with_stub_engines(tmp_path, monkeypatch):
         M.Qwen3TTSTokenizer.from_pretrained(str(tmp_path / "speech_tokenizer"), device_map="cpu")
 
 
-@pytest.mark.reference
 def test_tokenizer_config_defaults_match_reference():
-    from oracle import ref_shims
-    ref_shims.install()
-    from qwen_tts.core.tokenizer_12hz.configuration_qwen3_tts_tokenizer_v2 import (Qwen3TTSTokenizerV2Config,
-                                                                                   Qwen3TTSTokenizerV2DecoderConfig)
     from qwen3_tts_b200 import checkpoint
-    d = Qwen3TTSTokenizerV2DecoderConfig()
+    R = _reference_configs()
     for k, v in checkpoint.DECODER_DEFAULTS.items():
-        assert getattr(d, k) == v, k
-    t = Qwen3TTSTokenizerV2Config()
+        assert R["decoder_defaults"][k] == v, k
     for k, v in checkpoint.TOKENIZER_DEFAULTS.items():
-        assert getattr(t, k) == v, k
+        assert R["tokenizer_defaults"][k] == v, k
     _, tok, _ = tiny_checkpoint_configs()
-    ref = Qwen3TTSTokenizerV2Config(**{k: v for k, v in tok.items() if k != "model_type"})
-    c1, e1, _ = checkpoint.tokenizer_configs_from_dict(ref.to_dict())
+    c1, e1, _ = checkpoint.tokenizer_configs_from_dict(R["tokenizer_to_dict"])
     c2, e2, _ = checkpoint.tokenizer_configs_from_dict(tok)
     assert dataclasses.asdict(c1) == dataclasses.asdict(c2) and dataclasses.asdict(e1) == dataclasses.asdict(e2)
 
