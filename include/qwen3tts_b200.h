@@ -203,6 +203,33 @@ int q3_codec_last_launch_count(q3_codec* c);
  * (:638-658).  stage < 0 clears all captures. */
 int q3_codec_debug_capture(q3_codec* c, int32_t stage, void* dst_dev, int64_t capacity);
 
+/* Test hook (tests/ only): one launch of the tcgen05 tap-GEMM that runs every codec Conv1d / ConvTranspose1d / Linear,
+ * the talker prefill GEMMs and the code-predictor projection table, planned exactly as those callers plan it:
+ *   C[b][m][n] = epilogue( sum_tap sum_k A[b][m + shifts[tap] + a_row0][k] * W[n][tap*Kp + k] ),
+ * rows outside [0, a_rows) reading as zero.  A: bf16 [B] rows of a_bs elements, each holding a_rows rows of K (row
+ * pitch K); W: bf16 [N][ntaps*Kp].  bn = 0 takes the production tile width (gemm_pick_bn); a_rows = 0 means T; batch
+ * strides of 0 mean contiguous [B][T][N] ([B][T][N/2] for the gated activations); cmod = 0 means N; max_ctas = 0 runs
+ * one CTA per SM.  act: 0 none, 1 SnakeBeta, 2 GELU, 3 SwiGLU (gate, up) column pairs, 4 SwiGLU blocks of 8 gate | 8 up.
+ * bias / scale / snake_ea (exp(alpha)) / snake_ib (1/(exp(beta)+1e-9)) are fp32 [cmod]; resid / out_raw / out_act
+ * bf16.  An invalid descriptor is refused with a message before anything is enqueued. */
+typedef struct {
+  const void* a;
+  int32_t B, T, K, a_rows, a_row0;
+  int64_t a_bs;
+  const void* w;
+  int32_t N, Kp, ntaps, shifts[8];
+  int32_t bn, act, cmod;
+  const float *bias, *scale, *snake_ea, *snake_ib;
+  const void* resid;
+  int64_t resid_bs;
+  void* out_raw;
+  int64_t raw_bs;
+  void* out_act;
+  int64_t act_bs;
+  int32_t max_ctas;
+} q3_tap_gemm_desc;
+int q3_debug_tap_gemm(const q3_tap_gemm_desc* d, void* stream);
+
 /* ---------------------------------------------------------------- codec ENCODER (Qwen3TTSTokenizer.encode)
  * Replaces Qwen3TTSTokenizerV2Model.encode (core/tokenizer_12hz/modeling_qwen3_tts_tokenizer_v2.py:961-991), i.e.
  * transformers MimiModel._encode_frame (modeling_mimi.py:1455-1488), restricted to the first

@@ -57,6 +57,16 @@ class SpkCfg(C.Structure):
                 ("win", C.c_int32), ("device", C.c_int32)]
 
 
+class TapGemmDesc(C.Structure):
+    """q3_tap_gemm_desc: one tap-GEMM launch through the test hook q3_debug_tap_gemm."""
+    _fields_ = [("a", C.c_void_p)] + [(n, C.c_int32) for n in ("B", "T", "K", "a_rows", "a_row0")] + \
+               [("a_bs", C.c_int64), ("w", C.c_void_p)] + [(n, C.c_int32) for n in ("N", "Kp", "ntaps")] + \
+               [("shifts", C.c_int32 * 8)] + [(n, C.c_int32) for n in ("bn", "act", "cmod")] + \
+               [(n, C.c_void_p) for n in ("bias", "scale", "snake_ea", "snake_ib", "resid")] + \
+               [("resid_bs", C.c_int64), ("out_raw", C.c_void_p), ("raw_bs", C.c_int64), ("out_act", C.c_void_p),
+                ("act_bs", C.c_int64), ("max_ctas", C.c_int32)]
+
+
 # every symbol include/qwen3tts_b200.h declares (tests/test_abi.py checks the header against this list)
 AR_SYMBOLS = ["q3_abi_version", "q3_last_error", "q3_engine_create", "q3_engine_destroy", "q3_engine_load_tensor",
               "q3_engine_finalize", "q3_prefill", "q3_decode", "q3_get_progress", "q3_set_debug",
@@ -64,6 +74,7 @@ AR_SYMBOLS = ["q3_abi_version", "q3_last_error", "q3_engine_create", "q3_engine_
               "q3_session_begin", "q3_admit", "q3_release_slots", "q3_append_trailing", "q3_set_hidden_capture"]
 CODEC_SYMBOLS = ["q3_codec_create", "q3_codec_destroy", "q3_codec_load_tensor", "q3_codec_finalize",
                  "q3_codec_forward", "q3_codec_total_upsample", "q3_codec_last_launch_count", "q3_codec_debug_capture",
+                 "q3_debug_tap_gemm",
                  "q3_codec_stream_open", "q3_codec_stream_step", "q3_codec_stream_reset", "q3_codec_stream_position", "q3_codec_stream_close",
                  "q3_codec_enc_create", "q3_codec_enc_destroy", "q3_codec_enc_load_tensor", "q3_codec_enc_finalize",
                  "q3_codec_enc_encode", "q3_codec_enc_frames", "q3_codec_enc_hop", "q3_codec_enc_last_launch_count",
@@ -135,6 +146,7 @@ def load():
         lib.q3_codec_total_upsample.argtypes = [vp]
         lib.q3_codec_last_launch_count.argtypes = [vp]
         lib.q3_codec_debug_capture.argtypes = [vp, i32, vp, i64]
+        lib.q3_debug_tap_gemm.argtypes = [C.POINTER(TapGemmDesc), vp]
         lib.q3_codec_enc_create.argtypes = [C.POINTER(CodecEncCfg), C.POINTER(vp)]
         lib.q3_codec_enc_destroy.argtypes = [vp]
         lib.q3_codec_enc_destroy.restype = None

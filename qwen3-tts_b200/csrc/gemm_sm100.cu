@@ -498,9 +498,11 @@ int gemm_pick_bn(int N, int mtiles, int B) {
   return N;  // N < 64 (multiple of 16)
 }
 
-int gemm_launch(const GemmPlan& plan, cudaStream_t stream) {
+int gemm_launch(const GemmPlan& plan, cudaStream_t stream, int max_ctas) {
   const long long total = (long long)((plan.T + BM - 1) / BM) * ((plan.N + plan.bn - 1) / plan.bn) * plan.B;
-  const int grid = (int)std::min<long long>(total, g_sm_count > 0 ? g_sm_count : 148);  // persistent: one CTA per SM walks the tiles
+  int ctas = g_sm_count > 0 ? g_sm_count : 148;  // persistent: one CTA per SM walks the tiles
+  if (max_ctas > 0) ctas = std::min(ctas, max_ctas);
+  const int grid = (int)std::min<long long>(total, ctas);
   static const bool trace = getenv("Q3_GEMM_TRACE") != nullptr;  // tools/codec_breakdown.py joins this with an ncu launch list
   if (trace)
     fprintf(stderr, "[tap_gemm] B=%d T=%d N=%d Kp=%d taps=%d bn=%d tiles=%lld act=%d resid=%d\n", plan.B, plan.T, plan.N, plan.Kp,
@@ -516,4 +518,41 @@ int gemm_launch(const GemmPlan& plan, cudaStream_t stream) {
   }
   Q3_CUDA(cudaGetLastError());
   return 0;
+}
+
+#include "../../include/qwen3tts_b200.h"
+
+// Test hook: one tap-GEMM launch through the production planning (gemm_make_plan_v, gemm_pick_bn) and launch path.  The
+// checks here cover only what the kernel would otherwise dereference blindly; gemm_make_plan_v refuses the rest.
+extern "C" int q3_debug_tap_gemm(const q3_tap_gemm_desc* d, void* stream) {
+  Q3_REQUIRE(d && d->a && d->w, "tap_gemm: null descriptor, A or W");
+  Q3_REQUIRE(d->B >= 1 && d->T >= 1 && d->K >= 1 && d->N >= 1, "tap_gemm: empty problem (B=%d T=%d K=%d N=%d)", d->B, d->T, d->K, d->N);
+  Q3_REQUIRE(d->act >= ACT_NONE && d->act <= ACT_SWIGLU_BLK8, "tap_gemm: unknown activation %d", d->act);
+  Q3_REQUIRE(d->bn >= 0 && d->max_ctas >= 0 && d->cmod >= 0 && d->a_rows >= 0 && d->a_row0 >= 0, "tap_gemm: negative field");
+  const bool gated = d->act == ACT_SWIGLU_PAIR || d->act == ACT_SWIGLU_BLK8;
+  Q3_REQUIRE(d->out_raw || d->out_act, "tap_gemm: no output");
+  Q3_REQUIRE(!gated || d->out_act, "tap_gemm: gated epilogues need out_act");
+  Q3_REQUIRE(d->act != ACT_SNAKE || !d->out_act || (d->snake_ea && d->snake_ib), "tap_gemm: SnakeBeta needs snake_ea and snake_ib");
+  // every store and residual load moves 16 bytes: outputs / residual and their batch strides must keep that alignment
+  Q3_REQUIRE((uintptr_t)d->out_raw % 16 == 0 && (uintptr_t)d->out_act % 16 == 0 && (uintptr_t)d->resid % 16 == 0 &&
+                 d->raw_bs % 8 == 0 && d->act_bs % 8 == 0 && d->resid_bs % 8 == 0,
+             "tap_gemm: outputs / residual must be 16-byte aligned with batch strides that are multiples of 8 elements");
+  if (gemm_init()) return 1;
+  GemmEpilogue ep{};
+  ep.bias = d->bias; ep.scale = d->scale; ep.resid = reinterpret_cast<const bf16*>(d->resid);
+  ep.snake_ea = d->snake_ea; ep.snake_ib = d->snake_ib;
+  ep.cmod = d->cmod ? d->cmod : d->N;
+  ep.act = d->act;
+  ep.out_raw = reinterpret_cast<bf16*>(d->out_raw); ep.out_act = reinterpret_cast<bf16*>(d->out_act);
+  GemmViews v;
+  v.a_rows = d->a_rows; v.a_row0 = d->a_row0;
+  v.raw_bs = d->raw_bs; v.act_bs = d->act_bs; v.resid_bs = d->resid_bs;
+  const int a_rows = d->a_rows ? d->a_rows : d->T;
+  const int64_t a_bs = d->a_bs ? d->a_bs : (int64_t)a_rows * d->K;
+  const int bn = d->bn ? d->bn : gemm_pick_bn(d->N, (d->T + BM - 1) / BM, d->B);
+  GemmPlan plan;
+  if (gemm_make_plan_v(&plan, reinterpret_cast<const bf16*>(d->a), d->B, d->T, d->K, d->K, a_bs, reinterpret_cast<const bf16*>(d->w),
+                       d->N, d->Kp, d->ntaps, d->shifts, bn, ep, v))
+    return 1;
+  return gemm_launch(plan, reinterpret_cast<cudaStream_t>(stream), d->max_ctas);
 }

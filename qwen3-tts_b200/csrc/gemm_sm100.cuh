@@ -48,6 +48,7 @@ int gemm_make_plan(GemmPlan* plan, const bf16* a, int B, int T, int K, int64_t l
                    const bf16* w, int N, int Kp, int ntaps, const int* shifts, int bn, const GemmEpilogue& ep);
 int gemm_make_plan_v(GemmPlan* plan, const bf16* a, int B, int T, int K, int64_t lda, int64_t a_batch_stride, const bf16* w,
                      int N, int Kp, int ntaps, const int* shifts, int bn, const GemmEpilogue& ep, const GemmViews& v);
-int gemm_launch(const GemmPlan& plan, cudaStream_t stream);
+// max_ctas > 0 caps the persistent grid below one CTA per SM (tests: more tiles per CTA on the same problem)
+int gemm_launch(const GemmPlan& plan, cudaStream_t stream, int max_ctas = 0);
 int gemm_init();  // resolves cuTensorMapEncodeTiled, sets kernel attributes
 int gemm_pick_bn(int N, int mtiles, int B);  // largest tile width that still fills the 148 SMs
